@@ -19,6 +19,8 @@ sampler_ref.py  restatement of noise_schedule / sample_sr / denoise /
 kernel_ref.py   per-kernel torch references of every C-ABI entry point
                 (what each CUDA kernel must compute, incl. its rounding points).
 make_golden.py  runs the real reference here and writes tests/golden/*.
+make_golden_reference.py  the same for the tests that compare the CogVideoX path, the UNet restatement
+                and the CLI boundary against the reference (CPU cases, and GPU cases on a B200).
 
 Parity status: UNet / sampler restatements are PINNED against the real
 reference modules executed in this container (tests/test_oracle_pinning.py,

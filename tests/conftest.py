@@ -15,7 +15,6 @@ def pytest_configure(config):
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
     config.addinivalue_line("markers", "gpu: needs a CUDA (sm_100) device")
-    config.addinivalue_line("markers", "reference: needs the reference tree at /root/reference (build container only)")
 
 
 def pytest_sessionstart(session):
@@ -30,10 +29,6 @@ def pytest_sessionstart(session):
 def pytest_collection_modifyitems(config, items):
     import torch
     has_gpu = torch.cuda.is_available()
-    from oracle.ref_loader import reference_available
-    has_ref = reference_available()
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="reference tree not present"))

@@ -3,7 +3,7 @@ STAR's layer_forward on top of sat's default leaf modules, which are not in the 
 import pytest
 import torch
 
-from tests.util import rel_l2
+from tests.util import load_golden, rel_l2, sample_flat
 
 
 def _setup(cfg_kw, seed=3):
@@ -60,68 +60,88 @@ def test_dit_layer_gpu(cfg_kw):
 
 # ------------------------------------------------------------------------------------------------------------------
 # Whole DiffusionTransformer (patch embed, text proj, time embed, N layers with LoRA, final LayerNorm, final layer,
-# unpatchify) against the REFERENCE'S OWN FILES executed behind the sat shim (oracle/cogvideox_sat.py).  Needs the
-# reference tree (/root/reference or the staged oracle/_ref): marker `reference`.
+# unpatchify) against outputs of the REFERENCE'S OWN FILES executed behind the sat shim (oracle/cogvideox_sat.py), stored
+# by oracle/make_golden_reference.py in tests/golden/reference_cpu.pt and reference_gpu.pt.
 SMALL_DIT = dict(num_layers=2, hidden_size=128, num_attention_heads=2, num_frames=9, latent_height=8, latent_width=12,
                  text_length=6, text_hidden_size=32, lora_r=8, time_embed_dim=64)
+FULL_WIDTH_DIT = dict(num_layers=2, hidden_size=3072, num_attention_heads=48, num_frames=9, latent_height=16, latent_width=20,
+                      text_length=226, text_hidden_size=4096, lora_r=64, time_embed_dim=512)
+# reference state-dict entries star_b200's DiffusionTransformer recomputes instead of loading (rope tables)
+DIT_DERIVED = ("mixins.pos_embed.freqs_", "transformer.position_embeddings.weight")
 
 
-def _dit_pair(kw, dtype, device, seed=4):
-    """(reference net with a synthetic non-zero state dict, star_b200 net with the same weights, inputs)"""
-    from oracle import cogvideox_sat as S
-    from star_b200.cogvideox import DiffusionTransformer
+def dit_weights(manifest, seed=4):
+    """synthetic non-zero weights for a DiffusionTransformer state-dict manifest {key: shape}"""
     from star_b200.utils.synth import synth_tensor
-    ref = S.build_reference_dit(**kw)
     sd = {}
-    for k, v in ref.state_dict().items():
-        if "freqs_" in k:
-            sd[k] = v
-            continue
-        t = synth_tensor(k, v.shape, seed)
+    for k, shape in manifest.items():
+        t = synth_tensor(k, shape, seed)
         if k.endswith("temp_local.conv1.weight") or k.endswith("spa_local.conv1.weight"):
             t = t * 0.5
         if ".matrix_B." in k:                              # LoRA B is zero-initialised by sat: make the merge matter
             t = t * 8.0
         sd[k] = t
-    ref.load_state_dict(sd)
-    ref = ref.to(device)
-    net = DiffusionTransformer(**kw, dtype=dtype)
-    net.load_state_dict(sd)
-    net = net.to(device)
+    return sd
+
+
+def dit_inputs(kw):
+    """seeded (x, timesteps, context) of one DiT call"""
     g = torch.Generator().manual_seed(1)
     frames = (kw["num_frames"] - 1) // 4 + 1
-    x = torch.randn(2, frames, 32, kw["latent_height"], kw["latent_width"], generator=g).to(device)
-    ctx = torch.randn(2, kw["text_length"], kw["text_hidden_size"], generator=g).to(device)
-    t = torch.tensor([731, 12]).to(device)
-    return ref, net, x, t, ctx
+    x = torch.randn(2, frames, 32, kw["latent_height"], kw["latent_width"], generator=g)
+    ctx = torch.randn(2, kw["text_length"], kw["text_hidden_size"], generator=g)
+    return x, torch.tensor([731, 12]), ctx
 
 
-@pytest.mark.reference
-def test_dit_model_host_graph_vs_reference_files(monkeypatch):
-    """CPU: star_b200's host graph (im2col patch embed, LoRA merge, adaLN folding, layer stack, final layer, unpatchify) on the
-    emulated kernels against the reference's unmodified DiffusionTransformer (sat shimmed)."""
+def dit_net(kw, dtype, device):
+    """star_b200 DiffusionTransformer with dit_weights"""
+    from star_b200.cogvideox import DiffusionTransformer
+    net = DiffusionTransformer(**kw, dtype=dtype)
+    net.load_state_dict(dit_weights({k: v.shape for k, v in net.state_dict().items()}))
+    return net.to(device)
+
+
+def _emulate(monkeypatch):
     from oracle import kernel_ref as KR
     from star_b200 import ops
     for name in dir(KR):
         if not name.startswith("_") and callable(getattr(KR, name)) and hasattr(ops, name):
             monkeypatch.setattr(ops, name, getattr(KR, name))
-    ref, net, x, t, ctx = _dit_pair(SMALL_DIT, torch.float16, "cpu")
-    want = ref(x, timesteps=t, context=ctx)
+
+
+def test_dit_model_host_graph_vs_reference_files(monkeypatch):
+    """CPU: star_b200's host graph (im2col patch embed, LoRA merge, adaLN folding, layer stack, final layer, unpatchify) on the
+    emulated kernels against the reference's unmodified DiffusionTransformer (sat shimmed); same state-dict layout."""
+    gold = load_golden("reference_cpu.pt")
+    _emulate(monkeypatch)
+    net = dit_net(SMALL_DIT, torch.float16, "cpu")
+    assert {k: tuple(v.shape) for k, v in net.state_dict().items()} == \
+           {k: s for k, s in gold["dit_manifest"].items() if not k.startswith(DIT_DERIVED)}
+    x, t, ctx = dit_inputs(SMALL_DIT)
     got = net(x, timesteps=t, context=ctx)
+    want = gold["dit_out"]
     assert got.shape == want.shape == (2, 3, 16, 8, 12)
     err = rel_l2(got, want)
     print(f"DiT model host graph vs reference files: rel-L2 {err:.3e}")
     assert err < 3e-3
 
 
-@pytest.mark.reference
+RESTATED_LAYER_DIT = dict(SMALL_DIT, num_layers=1, lora_r=0)
+
+
+def restated_layer_inputs():
+    """(hidden, emb) of the one-layer check below: text 6 + 3 x 4 x 6 patches, hidden 128"""
+    g = torch.Generator().manual_seed(2)
+    return torch.randn(2, 6 + 72, 128, generator=g), torch.randn(2, 64, generator=g)
+
+
 def test_restated_layer_oracle_is_pinned_to_reference_files():
     """oracle/cogvideox_ref.py (the line-by-line restatement the layer tests use) == the reference's layer_forward"""
     from oracle.cogvideox_ref import DiTCfg, dit_layer_forward
-    from star_b200.cogvideox import rope_tables
-    kw = dict(SMALL_DIT, num_layers=1, lora_r=0)
-    ref, _, x, t, ctx = _dit_pair(kw, torch.float16, "cpu")
-    sd = ref.state_dict()
+    from star_b200.cogvideox import DiffusionTransformer, rope_tables
+    with torch.device("meta"):
+        manifest = {k: v.shape for k, v in DiffusionTransformer(**RESTATED_LAYER_DIT, dtype=torch.float16).state_dict().items()}
+    sd = dit_weights(manifest)
     cfg = DiTCfg(hidden=128, heads=2, text_length=6, frames=3, height=4, width=6)
     lsd = {"adaLN_modulation.1.weight": sd["mixins.adaln_layer.adaLN_modulations.0.1.weight"],
            "adaLN_modulation.1.bias": sd["mixins.adaln_layer.adaLN_modulations.0.1.bias"]}
@@ -131,31 +151,21 @@ def test_restated_layer_oracle_is_pinned_to_reference_files():
     for n in ("query", "key"):
         lsd[n + "_layernorm.weight"] = sd[f"mixins.adaln_layer.{n}_layernorm_list.0.weight"]
         lsd[n + "_layernorm.bias"] = sd[f"mixins.adaln_layer.{n}_layernorm_list.0.bias"]
-    g = torch.Generator().manual_seed(2)
-    hidden, emb = torch.randn(2, 6 + 72, 128, generator=g), torch.randn(2, 64, generator=g)
+    hidden, emb = restated_layer_inputs()
     cos, sin = rope_tables(3, 4, 6, 64)
-    ref.transformer.hooks.clear()
-    ref.transformer.hooks.update(ref.hooks)              # what BaseModel.forward does before every call
-    want = ref.hooks["layer_forward"](hidden, torch.ones(1, 1), layer_id=0, emb=emb, text_length=6)
     got = dit_layer_forward(lsd, hidden, emb, cfg, cos, sin)
-    assert rel_l2(got, want) < 1e-5
+    assert rel_l2(sample_flat(got), load_golden("reference_cpu.pt")["dit_layer_out"]) < 1e-5
 
 
 @pytest.mark.gpu
-@pytest.mark.reference
 @pytest.mark.parametrize("dtype,tol", [(torch.float16, 4e-3), (torch.bfloat16, 2.5e-2)])
 def test_dit_model_gpu_vs_reference_files(dtype, tol):
     """GPU: the whole (reduced-depth, full-width) DiT on the fp16 and bf16 kernel libraries vs the reference files in fp32;
-    the reference's own low-precision path (module.to(dtype), as sample_sr.py runs it) is measured beside it."""
-    kw = dict(num_layers=2, hidden_size=3072, num_attention_heads=48, num_frames=9, latent_height=16, latent_width=20,
-              text_length=226, text_hidden_size=4096, lora_r=64, time_embed_dim=512)
-    ref, net, x, t, ctx = _dit_pair(kw, dtype, "cuda")
-    want = ref(x, timesteps=t, context=ctx).float()
-    got = net(x, timesteps=t, context=ctx).float()
-    torch.cuda.synchronize()
-    ref_lp = ref.to(dtype)
-    ref_lp.dtype = dtype
-    low = ref_lp(x.to(dtype), timesteps=t, context=ctx.to(dtype)).float()
-    err, err_ref = rel_l2(got, want), rel_l2(low, want)
+    the error of the reference's own low-precision path (module.to(dtype), as sample_sr.py runs it) on the B200 bounds it."""
+    gold = load_golden("reference_gpu.pt")["dit"]
+    net = dit_net(FULL_WIDTH_DIT, dtype, "cuda")
+    x, t, ctx = (v.cuda() for v in dit_inputs(FULL_WIDTH_DIT))
+    got = net(x, timesteps=t, context=ctx).float().cpu()
+    err, err_ref = rel_l2(sample_flat(got), gold["out"]), gold["err_ref"][str(dtype)]
     print(f"DiT model [{dtype}] 2 layers x 3072: rel-L2 vs reference fp32 {err:.3e} (reference's own {dtype} path: {err_ref:.3e})")
     assert torch.isfinite(got).all() and err < tol and err < 2.0 * err_ref + 1e-3

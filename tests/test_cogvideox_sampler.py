@@ -1,9 +1,9 @@
-"""CogVideoX sampling loop (VPSDEDPMPP2MSampler + DynamicCFG + DiscreteDenoiser / VideoScaling) against the reference's UNMODIFIED
-sgm/modules/diffusionmodules files (oracle/cogvideox_sampler.py)."""
+"""CogVideoX sampling loop (VPSDEDPMPP2MSampler + DynamicCFG + DiscreteDenoiser / VideoScaling) against outputs of the reference's
+UNMODIFIED sgm/modules/diffusionmodules files (oracle/cogvideox_sampler.py), stored by oracle/make_golden_reference.py."""
 import pytest
 import torch
 
-from tests.util import rel_l2
+from tests.util import load_golden, rel_l2, sample_flat
 
 
 class FakeDiT(torch.nn.Module):
@@ -21,43 +21,32 @@ class FakeDiT(torch.nn.Module):
         return torch.tanh(0.8 * noisy - 0.3 * lq + 0.1 * noisy.mean(dim=1, keepdim=True)) * (1.0 + 0.2 * c) + 0.05 * t * lq
 
 
-@pytest.mark.reference
 def test_step_plan_matches_reference_tables():
-    from oracle.cogvideox_sampler import build_reference_sampler
     from star_b200.cogvideox.sampling import StepPlan
-    sampler, denoiser = build_reference_sampler()
-    x = torch.zeros(1, 2, 16, 4, 4)
-    _, s_in, acs, num_sigmas, _, _, timesteps = sampler.prepare_sampling_loop(x, {}, None, None)
+    gold, tables = load_golden("reference_cpu.pt")["sampler"], load_golden("cogvideox_path.pt")
+    acs, timesteps = tables["acs"], tables["timesteps"]
     plan = StepPlan()
-    assert num_sigmas == 51 and torch.equal(plan.alphas_cumprod_sqrt, acs)
-    assert plan.timesteps == [int(t) for t in timesteps]
+    assert gold["num_sigmas"] == 51 and torch.equal(plan.alphas_cumprod_sqrt, acs)
+    assert plan.timesteps == timesteps
     for i, st in enumerate(plan.steps):                                   # quantised sigma of the denoiser, guidance scale
-        q = denoiser.possibly_quantize_sigma(acs[i:i + 1])
-        assert st.c_skip == float(q) and st.timestep == int(timesteps[-(i + 1)])
-        assert st.cfg_scale == sampler.guider.scale_schedule(None, 50 - st.timestep)
+        assert st.c_skip == float(tables["sigma_q"][i]) and st.timestep == timesteps[-(i + 1)]
+        assert st.cfg_scale == tables["cfg"][i]
     assert [st.last for st in plan.steps] == [False] * 49 + [True]
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("steps", [50, 6])
 def test_sampler_matches_reference(steps):
-    from oracle.cogvideox_sampler import build_reference_sampler, reference_sample
+    from oracle.make_golden_cogvideox import sampler_inputs
     from star_b200.cogvideox.sampling import VPSDEDPMPP2MSampler
-    g = torch.Generator().manual_seed(0)
-    lq = torch.randn(1, 3, 16, 6, 8, generator=g)
-    randn = torch.randn(1, 3, 16, 6, 8, generator=g)
-    cond = {"crossattn": torch.randn(1, 226, 32, generator=g)}
-    uc = {"crossattn": torch.zeros(1, 226, 32)}
-    ref_sampler, ref_den = build_reference_sampler(num_steps=steps)
-    net_r, net_m = FakeDiT(), FakeDiT()
-    torch.manual_seed(123)
-    want = reference_sample(net_r, ref_sampler, ref_den, randn.clone(), dict(cond), dict(uc), lq)
+    gold = load_golden("reference_cpu.pt")["sampler"]["runs"][steps]
+    lq, randn, cond, uc = sampler_inputs()
+    net_m = FakeDiT()
     mine = VPSDEDPMPP2MSampler(num_steps=steps, dtype=torch.float32)
     torch.manual_seed(123)
     got = mine(net_m, randn.clone(), cond, uc=uc, lq=torch.cat((lq, lq), 0))
-    assert net_m.calls == net_r.calls and len(net_m.calls) == steps
-    assert got.shape == want.shape == randn.shape
-    assert rel_l2(got, want) < 2e-5
+    assert net_m.calls == gold["calls"] and len(net_m.calls) == steps
+    assert got.shape == gold["out"].shape == randn.shape
+    assert rel_l2(got, gold["out"]) < 2e-5
     # random-stream consumption: 1 draw in the first step, 2 in every later one but the last (sampling.py:635,:641)
     after = torch.randn(4)
     torch.manual_seed(123)
@@ -66,36 +55,19 @@ def test_sampler_matches_reference(steps):
     assert torch.equal(after, torch.randn(4))
 
 
-def _pipeline_pair(dit_kw, vae_kw, dtype, device):
-    from tests.test_cogvideox import _dit_pair
-    from tests.test_cogvideox_vae import _enc_pair, _pair
-    ref_dit, net, _x, _t, ctx = _dit_pair(dit_kw, dtype, device)
-    ref_dec, dec, _ = _pair(vae_kw, device=device, dtype=dtype)
-    ref_enc, enc, _ = _enc_pair(vae_kw, device=device, dtype=dtype)
-    return ref_dit, net, (ref_enc, ref_dec), (enc, dec), ctx
+def pipeline_nets(dit_kw, vae_kw, dtype, device):
+    """star_b200 DiT, 3-D VAE encoder / decoder with the weights of the stored reference runs, and the text context"""
+    from tests.test_cogvideox import dit_inputs, dit_net
+    from tests.test_cogvideox_vae import _decoder, _encoder
+    return dit_net(dit_kw, dtype, device), _encoder(vae_kw, device=device, dtype=dtype), \
+        _decoder(vae_kw, device=device, dtype=dtype), dit_inputs(dit_kw)[2].to(device)
 
 
-def _reference_pipeline(ref_dit, ref_vae, cond, uc, lq, steps, seed, scale_factor=0.7):
-    """sample_sr.py:186-230 / diffusion_video.py:245-292 on the reference's own modules (3-D VAE encoder + Gaussian posterior sample,
-    DiT behind the sat shim, sampler stack, 3-D VAE decoder); lq (1, F, 3, H, W)"""
-    from oracle.cogvideox_sampler import build_reference_sampler, reference_sample
-    from oracle.cogvideox_vae import load_reference_vae, reference_decode_latent, reference_encode_moments
-    ref_enc, ref_dec = ref_vae
-    sampler, den = build_reference_sampler(num_steps=steps, device=str(lq.device))
-    torch.manual_seed(seed)
-    F, H, W = lq.shape[1], lq.shape[3], lq.shape[4]
-    randn = torch.randn((1, (F - 1) // 4 + 1, 16, H // 8, W // 8), dtype=torch.float32).to(lq.device)
-    moments = reference_encode_moments(ref_enc, lq.permute(0, 2, 1, 3, 4).contiguous())
-    mean, logvar = torch.chunk(moments, 2, dim=1)                         # DiagonalGaussianDistribution.sample (regularizers.py:10-29)
-    zq = mean + torch.exp(0.5 * torch.clamp(logvar, -30.0, 20.0)) * torch.randn_like(mean)
-    lq_latent = (scale_factor * zq).permute(0, 2, 1, 3, 4).contiguous()
-    z = reference_sample(ref_dit, sampler, den, randn, dict(cond), dict(uc), lq_latent)
-    latent = (1.0 / scale_factor) * z.permute(0, 2, 1, 3, 4).contiguous()
-    frames = reference_decode_latent(ref_dec, latent).float().permute(0, 2, 1, 3, 4)
-    return torch.clamp((frames + 1.0) / 2.0, 0.0, 1.0), z
+def pipeline_lq(F, H, W):
+    """LQ clip (1, F, 3, H, W), already upsampled"""
+    return torch.rand(1, F, 3, H, W, generator=torch.Generator().manual_seed(9)) * 2 - 1
 
 
-@pytest.mark.reference
 def test_cogvideox_pipeline_host_graph_on_emulated_kernels(monkeypatch):
     """LQ frames -> frames through 3-D VAE encode + DiT + sampler + 3-D VAE decode (reduced sizes, 4 steps) against the same chain of
     reference modules"""
@@ -104,37 +76,32 @@ def test_cogvideox_pipeline_host_graph_on_emulated_kernels(monkeypatch):
     from star_b200.cogvideox import sample_sr
     from tests.test_cogvideox import SMALL_DIT
     from tests.test_cogvideox_vae import SMALL
+    gold = load_golden("reference_cpu.pt")["pipeline"]
     for name in dir(KR):
         if not name.startswith("_") and callable(getattr(KR, name)) and hasattr(ops, name):
             monkeypatch.setattr(ops, name, getattr(KR, name))
-    ref_dit, net, ref_vae, (enc, dec), ctx = _pipeline_pair(SMALL_DIT, SMALL, torch.float16, "cpu")
+    net, enc, dec, ctx = pipeline_nets(SMALL_DIT, SMALL, torch.float16, "cpu")
     cond, uc = {"crossattn": ctx[:1]}, {"crossattn": torch.zeros_like(ctx[:1])}
-    lq = torch.rand(1, 9, 3, 64, 96, generator=torch.Generator().manual_seed(9)) * 2 - 1          # LQ clip, already upsampled
-    want, z_ref = _reference_pipeline(ref_dit, ref_vae, cond, uc, lq, steps=4, seed=77)
-    got, z = sample_sr(net, dec, cond, uc, lq=lq, encoder=enc, num_steps=4, seed=77)
-    assert got.shape == want.shape == (1, 9, 3, 64, 96)
-    assert rel_l2(z, z_ref) < 1e-2 and rel_l2(got, want) < 1e-2
+    got, z = sample_sr(net, dec, cond, uc, lq=pipeline_lq(9, 64, 96), encoder=enc, num_steps=4, seed=77)
+    assert got.shape == (1, 9, 3, 64, 96)
+    assert rel_l2(sample_flat(z), gold["z"]) < 1e-2 and rel_l2(sample_flat(got), gold["frames"]) < 1e-2
+
+
+FULL_WIDTH_PIPELINE_DIT = dict(num_layers=2, hidden_size=3072, num_attention_heads=48, num_frames=17, latent_height=16, latent_width=24,
+                               text_length=226, text_hidden_size=4096, lora_r=64, time_embed_dim=512)
 
 
 @pytest.mark.gpu
-@pytest.mark.reference
 def test_cogvideox_pipeline_gpu():
     """the same chain on the B200 kernels: full-width DiT (2 layers), full-width 3-D VAE decoder, 6 sampler steps, fp16"""
-    from oracle.cogvideox_vae import vae_reference_available
-    from oracle.cogvideox_sampler import sampler_reference_available
     from star_b200.cogvideox import sample_sr
-    if not (vae_reference_available() and sampler_reference_available()):
-        pytest.skip("reference files not staged")
-    kw = dict(num_layers=2, hidden_size=3072, num_attention_heads=48, num_frames=17, latent_height=16, latent_width=24,
-              text_length=226, text_hidden_size=4096, lora_r=64, time_embed_dim=512)
-    ref_dit, net, ref_vae, (enc, dec), ctx = _pipeline_pair(kw, {}, torch.float16, "cuda")
+    gold = load_golden("reference_gpu.pt")["pipeline"]
+    net, enc, dec, ctx = pipeline_nets(FULL_WIDTH_PIPELINE_DIT, {}, torch.float16, "cuda")
     cond, uc = {"crossattn": ctx[:1]}, {"crossattn": torch.zeros_like(ctx[:1])}
-    lq = (torch.rand(1, 17, 3, 128, 192, generator=torch.Generator().manual_seed(9)) * 2 - 1).cuda()
-    want, z_ref = _reference_pipeline(ref_dit, ref_vae, cond, uc, lq, steps=6, seed=5)
-    got, z = sample_sr(net, dec, cond, uc, lq=lq, encoder=enc, num_steps=6, seed=5)
-    e_z, e_x = rel_l2(z, z_ref), rel_l2(got, want)
+    got, z = sample_sr(net, dec, cond, uc, lq=pipeline_lq(17, 128, 192).cuda(), encoder=enc, num_steps=6, seed=5)
+    e_z, e_x = rel_l2(sample_flat(z), gold["z"]), rel_l2(sample_flat(got), gold["frames"])
     print(f"[cogvideox pipeline fp16, 6 steps] latent rel-L2 {e_z:.2e}, frames rel-L2 {e_x:.2e}")
-    assert got.shape == want.shape == (1, 17, 3, 128, 192) and torch.isfinite(got).all()
+    assert got.shape == (1, 17, 3, 128, 192) and torch.isfinite(got).all()
     assert e_z < 2e-2 and e_x < 2e-2
 
 

@@ -1,38 +1,44 @@
-"""CogVideoX 3-D causal VAE decoder (SURVEY 8 row f4) against the reference's UNMODIFIED cp_enc_dec.py
-(oracle/cogvideox_vae.py: context-parallel size 1, SafeConv3d = Conv3d)."""
+"""CogVideoX 3-D causal VAE decoder (SURVEY 8 row f4) against outputs of the reference's UNMODIFIED cp_enc_dec.py
+(oracle/cogvideox_vae.py: context-parallel size 1, SafeConv3d = Conv3d), stored by oracle/make_golden_reference.py."""
 import pytest
 import torch
 
-from tests.util import assert_close, rel_l2
+from star_b200.utils.synth import synth_state_dict
+from tests.util import assert_close, load_golden, rel_l2, sample_flat
 
 SMALL = dict(ch=32, ch_mult=(1, 2, 2, 4), num_res_blocks=1)          # 32..128 channels, same topology as the shipped decoder
 
 
-def _pair(kw, seed=3, device="cpu", dtype=torch.float16):
-    from oracle.cogvideox_vae import build_reference_decoder
-    from star_b200.cogvideox.vae3d import ContextParallelDecoder3D
-    from star_b200.utils.synth import synth_state_dict
-    ref = build_reference_decoder(**kw)
-    sd = synth_state_dict({k: tuple(v.shape) for k, v in ref.state_dict().items()}, seed=seed)
+def decoder_weights(manifest, seed=3):
+    sd = synth_state_dict(manifest, seed=seed)
     for k in sd:                                    # conv_y multiplies the normalised features: keep it O(1), not O(1/sqrt(16))
         if ".conv_y.conv.bias" in k:
             sd[k] = sd[k] + 1.0
-    ref.load_state_dict(sd)
+    return sd
+
+
+def _decoder(kw, device="cpu", dtype=torch.float16):
+    from star_b200.cogvideox.vae3d import ContextParallelDecoder3D
     mine = ContextParallelDecoder3D(**kw)
-    mine.load_state_dict(sd)
-    return ref.to(device), mine.to(device=device, dtype=dtype).eval(), sd
+    mine.load_state_dict(decoder_weights({k: tuple(v.shape) for k, v in mine.state_dict().items()}))
+    return mine.to(device=device, dtype=dtype).eval()
 
 
-def _enc_pair(kw, seed=6, device="cpu", dtype=torch.float16):
-    from oracle.cogvideox_vae import build_reference_encoder
+def _encoder(kw, seed=6, device="cpu", dtype=torch.float16):
     from star_b200.cogvideox.vae3d import ContextParallelEncoder3D
-    from star_b200.utils.synth import synth_state_dict
-    ref = build_reference_encoder(**kw)
-    sd = synth_state_dict({k: tuple(v.shape) for k, v in ref.state_dict().items()}, seed=seed)
-    ref.load_state_dict(sd)
     mine = ContextParallelEncoder3D(**kw)
-    mine.load_state_dict(sd)
-    return ref.to(device), mine.to(device=device, dtype=dtype).eval(), sd
+    mine.load_state_dict(synth_state_dict({k: tuple(v.shape) for k, v in mine.state_dict().items()}, seed=seed))
+    return mine.to(device=device, dtype=dtype).eval()
+
+
+def decoder_host_input():
+    return torch.randn(1, 16, 7, 4, 6, generator=torch.Generator().manual_seed(0))
+
+
+def encoder_host_inputs():
+    x = torch.rand(1, 3, 9, 32, 48, generator=torch.Generator().manual_seed(3)) * 2 - 1
+    even = torch.rand(1, 3, 8, 16, 16, generator=torch.Generator().manual_seed(4)) * 2 - 1      # even T: plain pair pooling
+    return x, even
 
 
 def _patch(monkeypatch):
@@ -43,57 +49,46 @@ def _patch(monkeypatch):
             monkeypatch.setattr(ops, name, getattr(KR, name))
 
 
-@pytest.mark.reference
 def test_state_dict_layout_matches_reference():
-    from oracle.cogvideox_vae import build_reference_decoder
     from star_b200.cogvideox.vae3d import ContextParallelDecoder3D
+    gold = load_golden("reference_cpu.pt")
     with torch.device("meta"):
         mine = ContextParallelDecoder3D()
-    ref = build_reference_decoder()
     got = {k: tuple(v.shape) for k, v in mine.state_dict().items()}
-    want = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
-    assert got == want
-    assert sum(torch.Size(s).numel() for s in got.values()) == sum(p.numel() for p in ref.parameters())
+    assert got == gold["vae_dec_manifest"]
+    assert sum(torch.Size(s).numel() for s in got.values()) == gold["vae_dec_params"]
 
 
-@pytest.mark.reference
 def test_decoder_host_graph_on_emulated_kernels(monkeypatch):
     """3 + 2 + 2 latent frames through the reference's chunk protocol (sample_sr.py:212-227): odd / even clip lengths, the
     first-frame split of SpatialNorm3D and Upsample3D, and the causal-conv context carried between chunks."""
-    from oracle.cogvideox_vae import reference_decode_latent
+    gold = load_golden("reference_cpu.pt")
     _patch(monkeypatch)
-    ref, mine, _ = _pair(SMALL)
-    z = torch.randn(1, 16, 7, 4, 6, generator=torch.Generator().manual_seed(0))
-    want = reference_decode_latent(ref, z)
+    mine = _decoder(SMALL)
+    z = decoder_host_input()
     got = mine.decode_latent(z)
-    assert got.shape == want.shape == (1, 3, 25, 32, 48) and got.dtype == torch.float16
-    assert rel_l2(got, want) < 3e-3
+    assert got.shape == (1, 3, 25, 32, 48) and got.dtype == torch.float16
+    assert rel_l2(sample_flat(got), gold["vae_dec_out"]) < 3e-3
     assert not mine._cache                                                    # the last chunk clears the context
     # a chunk decoded alone (clear cache) replicates its first frame instead of using context
-    with __import__("oracle.cogvideox_vae", fromlist=["single_rank"]).single_rank():
-        alone = ref(z[:, :, 3:5].contiguous(), clear_fake_cp_cache=True)
-    assert rel_l2(mine(z[:, :, 3:5].contiguous()), alone) < 3e-3
-    assert rel_l2(got[:, :, 9:17], alone) > 1e-2                              # ... and that differs from the chunked result
+    assert rel_l2(sample_flat(mine(z[:, :, 3:5].contiguous())), gold["vae_dec_alone"]) < 3e-3
+    assert rel_l2(sample_flat(got[:, :, 9:17]), gold["vae_dec_alone"]) > 1e-2  # ... and that differs from the chunked result
 
 
-@pytest.mark.reference
 def test_encoder_host_graph_on_emulated_kernels(monkeypatch):
     """9 frames of 32x48 -> moments (1, 32, 3, 4, 6): odd clip lengths through both time-compressing DownSample3D levels
     (9 -> 5 -> 3), the (0,1,0,1)-padded stride-2 convs, clip-wide GroupNorm, first-frame replication of the causal convs"""
-    from oracle.cogvideox_vae import build_reference_encoder, reference_encode_moments
     from star_b200.cogvideox.vae3d import ContextParallelEncoder3D
+    gold = load_golden("reference_cpu.pt")
     _patch(monkeypatch)
     with torch.device("meta"):
-        assert {k: tuple(v.shape) for k, v in ContextParallelEncoder3D().state_dict().items()} == \
-               {k: tuple(v.shape) for k, v in build_reference_encoder().state_dict().items()}
-    ref, mine, _ = _enc_pair(SMALL)
-    x = torch.rand(1, 3, 9, 32, 48, generator=torch.Generator().manual_seed(3)) * 2 - 1
-    want = reference_encode_moments(ref, x)
+        assert {k: tuple(v.shape) for k, v in ContextParallelEncoder3D().state_dict().items()} == gold["vae_enc_manifest"]
+    mine = _encoder(SMALL)
+    x, even = encoder_host_inputs()
     got = mine(x)
-    assert got.shape == want.shape == (1, 32, 3, 4, 6)
-    assert rel_l2(got, want) < 3e-3
-    even = torch.rand(1, 3, 8, 16, 16, generator=torch.Generator().manual_seed(4)) * 2 - 1      # even T: plain pair pooling
-    assert rel_l2(mine(even), reference_encode_moments(ref, even)) < 3e-3
+    assert got.shape == gold["vae_enc_out"].shape == (1, 32, 3, 4, 6)
+    assert rel_l2(got, gold["vae_enc_out"]) < 3e-3
+    assert rel_l2(mine(even), gold["vae_enc_even_out"]) < 3e-3
     torch.manual_seed(0)
     z = mine.encode(x)
     torch.manual_seed(0)
@@ -159,22 +154,20 @@ def test_groupnorm_mod(env, T, Tl, H, W, Hl, Wl, C):
     assert_close(got, KR.groupnorm_mod(x, gam, bet, mod[:, :C], mod[:, C:], T, H, W, Tl, Hl, Wl, 1e-6, True), what="groupnorm_mod")
 
 
+def decoder_gpu_input():
+    return torch.randn(1, 16, 5, 16, 24, generator=torch.Generator().manual_seed(1))
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("dtype,tol", [(torch.float16, 3e-3), (torch.bfloat16, 1.6e-2)])
 def test_decoder_vs_reference_gpu(dtype, tol):
     """full-width decoder (ch 128, 3 res blocks per level), 3 + 2 latent frames at 16x24 -> 17 frames of 128x192, against the
-    reference's own file in fp32 (TF32 off) and beside the reference run in the same 16-bit dtype"""
-    from oracle.cogvideox_vae import reference_decode_latent, vae_reference_available
-    if not vae_reference_available():
-        pytest.skip("reference VAE file not staged (oracle/_ref)")
-    ref, mine, sd = _pair({}, device="cuda", dtype=dtype)
-    z = torch.randn(1, 16, 5, 16, 24, generator=torch.Generator().manual_seed(1)).cuda()
-    want = reference_decode_latent(ref, z)
-    got = mine.decode_latent(z.to(dtype))
-    assert got.shape == want.shape == (1, 3, 17, 128, 192)
-    err = rel_l2(got, want)
-    ref16 = reference_decode_latent(ref.to(dtype), z.to(dtype))
-    err_ref = rel_l2(ref16, want)
+    reference's own file in fp32 (TF32 off) and beside the reference run in the same 16-bit dtype, both on the B200"""
+    gold = load_golden("reference_gpu.pt")["vae_dec"]
+    mine = _decoder({}, device="cuda", dtype=dtype)
+    got = mine.decode_latent(decoder_gpu_input().cuda().to(dtype))
+    assert got.shape == (1, 3, 17, 128, 192)
+    err, err_ref = rel_l2(sample_flat(got), gold["out"]), gold["err_ref"][str(dtype)]
     print(f"[cogvideox vae {dtype}] star {err:.2e}  reference-in-{dtype} {err_ref:.2e}")
     assert torch.isfinite(got.float()).all()
     assert err < tol and err < 1.5 * err_ref + 1e-3
@@ -189,19 +182,18 @@ def test_time_avgpool2(env, T, HW, C):
     assert got.shape == want.shape and torch.equal(got, want)                  # one rounding of an exact fp32 sum
 
 
+def encoder_gpu_input():
+    return torch.rand(1, 3, 17, 96, 128, generator=torch.Generator().manual_seed(2)) * 2 - 1
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("dtype,tol", [(torch.float16, 3e-3), (torch.bfloat16, 1.6e-2)])
 def test_encoder_vs_reference_gpu(dtype, tol):
     """full-width encoder (ch 128, 3 res blocks per level), 17 frames of 96x128 -> moments (1, 32, 5, 12, 16)"""
-    from oracle.cogvideox_vae import reference_encode_moments, vae_reference_available
-    if not vae_reference_available():
-        pytest.skip("reference VAE file not staged (oracle/_ref)")
-    ref, mine, _ = _enc_pair({}, device="cuda", dtype=dtype)
-    x = (torch.rand(1, 3, 17, 96, 128, generator=torch.Generator().manual_seed(2)) * 2 - 1).cuda()
-    want = reference_encode_moments(ref, x)
-    got = mine(x.to(dtype))
-    err = rel_l2(got, want)
-    err_ref = rel_l2(reference_encode_moments(ref.to(dtype), x.to(dtype)), want)
+    gold = load_golden("reference_gpu.pt")["vae_enc"]
+    mine = _encoder({}, device="cuda", dtype=dtype)
+    got = mine(encoder_gpu_input().cuda().to(dtype))
+    err, err_ref = rel_l2(sample_flat(got), gold["out"]), gold["err_ref"][str(dtype)]
     print(f"[cogvideox vae encoder {dtype}] star {err:.2e}  reference-in-{dtype} {err_ref:.2e}")
-    assert got.shape == want.shape == (1, 32, 5, 12, 16) and torch.isfinite(got.float()).all()
+    assert got.shape == (1, 32, 5, 12, 16) and torch.isfinite(got.float()).all()
     assert err < tol and err < 1.5 * err_ref + 1e-3

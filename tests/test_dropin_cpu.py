@@ -1,67 +1,28 @@
 """Drop-in check of the package-level boundary (INTEGRATION.md 1): the reference's own CLI module
-video_super_resolution/scripts/inference_sr.py, unmodified, imported with `video_to_video` aliased to
-star_b200.video_to_video, builds its STAR wrapper on star_b200's VideoToVideo_sr and calls test() with arguments the
-star_b200 signature accepts."""
-import importlib.util
+video_super_resolution/scripts/inference_sr.py, unmodified, was run with `video_to_video` aliased to star_b200.video_to_video
+and an in-memory clip (oracle/make_golden_reference.py); the calls it made into VideoToVideo_sr are stored in
+tests/golden/reference_cli_calls.json and must bind to star_b200's signatures."""
 import inspect
+import json
 import os
-import sys
+import types
 
-import pytest
-import torch
-
-REF = "/root/reference"
-SUBS = ("video_to_video_model", "diffusion", "diffusion.diffusion_sdedit", "diffusion.solvers_sdedit", "diffusion.schedules_sdedit",
-        "modules", "modules.unet_v2v", "utils", "utils.config", "utils.logger", "utils.seed")
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_cli_calls.json")
 
 
-@pytest.mark.reference
-def test_reference_cli_runs_on_star_b200(monkeypatch, tmp_path):
-    pytest.importorskip("cv2")
-    pytest.importorskip("torchvision")
-    from oracle import ref_loader                                   # easydict & co. shims only (test infrastructure)
-    ref_loader._install_shims()
-    import star_b200.video_to_video as v2v
-    saved = {k: v for k, v in sys.modules.items() if k == "video_to_video" or k.startswith("video_to_video.")}
-    for k in saved:
-        monkeypatch.delitem(sys.modules, k)
-    monkeypatch.setitem(sys.modules, "video_to_video", v2v)
-    for sub in SUBS:
-        mod = importlib.import_module("star_b200.video_to_video." + sub)
-        monkeypatch.setitem(sys.modules, "video_to_video." + sub, mod)
-    monkeypatch.syspath_prepend(REF)                                 # inference_utils.py, video_super_resolution/color_fix.py
+def test_reference_cli_runs_on_star_b200():
     from star_b200.video_to_video.video_to_video_model import VideoToVideo_sr
+    calls = json.load(open(GOLD))
+    init, test = calls["init"], calls["test"]
+    opt = types.SimpleNamespace(**init["opt"])
+    assert opt.model_path == "light_deg.pt" and not init["kwargs"]
+    inspect.signature(VideoToVideo_sr.__init__).bind(None, opt, *init["args"])
 
-    calls = {}
-
-    def fake_init(self, opt, device=torch.device("cuda:0"), **kw):
-        calls["opt"] = opt
-        self.positive_prompt, self.negative_prompt = ", good", "bad"
-
-    def fake_test(self, input, total_noise_levels=1000, steps=50, solver_mode="fast", guide_scale=7.5, max_chunk_len=32):
-        calls["test"] = dict(total_noise_levels=total_noise_levels, steps=steps, solver_mode=solver_mode,
-                             guide_scale=guide_scale, max_chunk_len=max_chunk_len, keys=sorted(input))
-        f, _, h, w = input["video_data"].shape
-        th, tw = input["target_res"]
-        return torch.zeros(1, 3, f, th, tw)
-
-    real_sig = inspect.signature(VideoToVideo_sr.test)
-    monkeypatch.setattr(VideoToVideo_sr, "__init__", fake_init)
-    monkeypatch.setattr(VideoToVideo_sr, "test", fake_test)
-    spec = importlib.util.spec_from_file_location("ref_inference_sr", os.path.join(REF, "video_super_resolution/scripts/inference_sr.py"))
-    cli = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(cli)                                     # the reference file itself, unmodified
-    assert cli.VideoToVideo_sr is VideoToVideo_sr
-    star = cli.STAR(result_dir=str(tmp_path), file_name="o.mp4", model_path="light_deg.pt", solver_mode="fast", steps=15)
-    assert isinstance(star.model, VideoToVideo_sr) and calls["opt"].model_path == "light_deg.pt"
-
-    # drive enhance_a_video with an in-memory clip (no codec / ffmpeg in the image): the reference's own pre/post run
-    frames = [(torch.rand(24, 32, 3) * 255).byte().numpy() for _ in range(3)]
-    monkeypatch.setattr(cli, "load_video", lambda path: (frames, 8.0))
-    monkeypatch.setattr(cli, "collate_fn", lambda data, device: data)            # no CUDA device in the build container
-    saved_out = {}
-    monkeypatch.setattr(cli, "save_video", lambda video, d, name, fps=16.0: saved_out.update(n=len(video), shape=tuple(video[0].shape)))
-    path = star.enhance_a_video("clip.mp4", "a cat")
-    assert path.endswith("o.mp4") and saved_out == {"n": 3, "shape": (96, 128, 3)}
-    assert calls["test"]["keys"] == ["target_res", "video_data", "y"] and calls["test"]["steps"] == 15
-    real_sig.bind(None, {"video_data": None}, 900, steps=15, solver_mode="fast", guide_scale=7.5, max_chunk_len=32)
+    assert test["input_keys"] == ["target_res", "video_data", "y"] and test["kwargs"]["steps"] == 15
+    video = test["input"]["video_data"]
+    assert video["shape"][0] == 3 and test["input"]["target_res"] == [96, 128]
+    inp = {"video_data": None, "y": test["input"]["y"], "target_res": tuple(test["input"]["target_res"])}
+    bound = inspect.signature(VideoToVideo_sr.test).bind(None, inp, *test["args"], **test["kwargs"])
+    assert bound.arguments["total_noise_levels"] == 900 and bound.arguments["solver_mode"] == "fast"
+    # the reference's own post-processing turned the (1, 3, F, 96, 128) result into F frames of 96x128x3
+    assert calls["saved"] == {"n": 3, "shape": [96, 128, 3]}

@@ -1,5 +1,5 @@
 """CPU suite (no GPU): the oracle against the golden vectors produced by the real reference
-(oracle/make_golden.py), and -- where /root/reference exists -- against the reference itself."""
+(oracle/make_golden.py, oracle/make_golden_reference.py)."""
 import json
 import os
 
@@ -31,37 +31,27 @@ def test_unet_restatement_matches_golden(small_sd):
         assert rel_l2(out, c["out_fp32"]) < 2e-5, c
 
 
-@pytest.mark.reference
-def test_unet_restatement_matches_live_reference(small_sd):
-    from oracle import ref_loader as R
-    from oracle.unet_ref import UNetCfg, controlled_unet_forward
-    U = R.load_reference().unet
-    with torch.device("meta"):
-        net = U.ControlledV2VUNet.__new__(U.ControlledV2VUNet)
-        U.Vid2VidSDUNet.__init__(net, **SMALL_KW)
-        net.VideoControlNet = U.VideoControlNet(**SMALL_KW)
-    net.load_state_dict(small_sd, assign=True)
-    net.eval()
+def live_reference_inputs():
     x, hint, y = make_inputs(42, 1, 3, 10, 16)
-    t = torch.tensor([123])
-    with torch.no_grad():
-        ref = net(x, t, y, hint=hint)
+    return x, torch.tensor([123]), y, hint
+
+
+def test_unet_restatement_matches_live_reference(small_sd):
+    """oracle/unet_ref.py (fp32) == the reference's own ControlledV2VUNet at a fourth input shape"""
+    from oracle.unet_ref import UNetCfg, controlled_unet_forward
+    x, t, y, hint = live_reference_inputs()
     out = controlled_unet_forward(small_sd, x, t, y, hint, UNetCfg(**SMALL_KW))
-    assert rel_l2(out, ref) < 2e-5
+    assert rel_l2(out, torch.load(os.path.join(GOLD, "reference_cpu.pt"))["unet_out"]) < 2e-5
 
 
-@pytest.mark.reference
 def test_state_dict_layout_matches_live_reference():
-    """2 247 tensors, same names and shapes as the reference's ControlledV2VUNet()."""
-    from oracle import ref_loader as R
+    """2 247 tensors, same names and shapes as the reference's ControlledV2VUNet() (manifest written from it)."""
     from star_b200.video_to_video.modules.unet_v2v import ControlledV2VUNet
-    U = R.load_reference().unet
+    man = json.load(open(os.path.join(GOLD, "state_dict_manifest.json")))
     with torch.device("meta"):
-        ref = U.ControlledV2VUNet()
         mine = ControlledV2VUNet()
-    a = {k: tuple(v.shape) for k, v in mine.state_dict().items()}
-    b = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
-    assert a == b and len(a) == 2247
+    a = {k: list(v.shape) for k, v in mine.state_dict().items()}
+    assert a == man and len(a) == 2247
 
 
 def test_state_dict_layout_matches_manifest():

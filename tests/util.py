@@ -17,6 +17,18 @@ def assert_close(got, ref, rel=2e-3, max_rel=2e-2, what=""):
     return e, m
 
 
+def sample_flat(t, n=4096, seed=0):
+    """A fixed, seeded sample of n elements of t (flattened): large golden outputs are stored as this sample."""
+    idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(seed))[:n]
+    return t.reshape(-1)[idx.to(t.device)].float().cpu()
+
+
+def load_golden(name):
+    """A golden file of tests/golden/ (outputs of the unmodified reference, see oracle/make_golden*.py)."""
+    import os
+    return torch.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name))
+
+
 SMALL_KW = dict(dim_mult=[1, 2, 1, 4], num_res_blocks=1)     # reduced ControlledV2VUNet used by fast tests
 
 
