@@ -12,26 +12,15 @@
 //   * two softmax threads per query row (640 threads): score columns [0,64) / [64,128) of the KV tile, O columns
 //     [0,32) / [32,64); the halves agree on the row maximum through shared memory and one 256-thread named barrier
 //     per KV tile.  16 softmax warps keep the 16-lane MUFU ~80 % busy (every exponential on the MUFU: the FMA-pipe
-//     polynomial share and the one-thread-per-row organisation were measured and lost, DESIGN.md section 3).
+//     polynomial share, the two query tiles taking turns on the MUFU and the one-thread-per-row organisation were
+//     measured and lost, DESIGN.md section 3).
 // TMEM columns: S[t] t*128, O[t] 256 + t*64, P[t] 384 + t*64.
 #pragma once
 #include "common.cuh"
 #include "attn.cuh"
 
-// Compile-time experiment knobs (tools/build_variant.py builds A/B libraries with -D...; the shipped library uses the
-// defaults below -- there is no run-time dispatch):
-//   STAR_ATTN_PINGPONG 1: the two query tiles' softmax groups take turns on the exponential phase (mbarrier token).  Both
-//                         tiles start together, and the 16-lane MUFU is a shared resource, so without the token they stay
-//                         in lock-step: both queue on the MUFU, then both sit in their MUFU-free phase (S wait, TMEM load,
-//                         row max, exchange, P store) -- the MUFU idles ~20 % of every KV step.
-//   STAR_ATTN_POLY n    : every n-th probability pair takes the FMA-pipe polynomial instead of MUFU.EX2 (0 = none).
-#ifndef STAR_ATTN_PINGPONG
-#define STAR_ATTN_PINGPONG 0
-#endif
-#ifndef STAR_ATTN_POLY
-#define STAR_ATTN_POLY 0
-#endif
-//   STAR_ATTN_TRACE 1   : CTA (0,0,0) records clock64() of the softmax phases of both tiles per KV step (tools/attn_trace.py).
+// Instrumented build (tools/build_variant.py -DSTAR_ATTN_TRACE=1; never set in the shipped library):
+//   STAR_ATTN_TRACE 1: CTA (0,0,0) records clock64() of the softmax phases of both tiles per KV step (tools/attn_trace.py).
 #ifndef STAR_ATTN_TRACE
 #define STAR_ATTN_TRACE 0
 #endif
@@ -93,8 +82,7 @@ attn4_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     uint64_t* s_free = bars + 13;            // 2   softmax WG t -> MMA : S_t(j) is in registers
     uint64_t* p_full = bars + 15;            // 2   softmax WG t -> MMA : P_t(j) in TMEM, O_t rescaled
     uint64_t* pv_done = bars + 17;           // 2   MMA -> softmax WG t : O_t += P_t(j) V_j retired
-    uint64_t* turn = bars + 19;              // 2   softmax group (1-t) -> group t : "your turn on the MUFU" (STAR_ATTN_PINGPONG)
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 21);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 19);
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
@@ -122,7 +110,6 @@ attn4_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 mbar_init(&s_free[t], 256);
                 mbar_init(&p_full[t], 256);
                 mbar_init(&pv_done[t], 1);
-                mbar_init(&turn[t], 256);
             }
             fence_barrier_init();
         }
@@ -301,27 +288,19 @@ attn4_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 uint64_t l0 = 0ull, l1 = 0ull;
                 uint32_t pk[32];
                 const uint64_t sl2_2 = f2_pack(sl2, sl2), negm_2 = f2_pack(-m_used, -m_used);
-                const bool pingpong = STAR_ATTN_PINGPONG && ntq == 2;
-                if (pingpong) mbar_wait(&turn[t], t == 0 ? ((j & 1) ^ 1) : (j & 1));
 #pragma unroll
                 for (int e = 0; e < 32; ++e) {
                     const int i = e * 2;
                     const uint64_t x01 = f2_fma(f2_pack_bits(v[i], v[i + 1]), sl2_2, negm_2);
-                    uint64_t p01;
-                    if (STAR_ATTN_POLY > 0 && (e % (STAR_ATTN_POLY > 0 ? STAR_ATTN_POLY : 1)) == STAR_ATTN_POLY - 1) {
-                        p01 = ex2_poly2(x01);
-                    } else {
-                        float x0, x1;
-                        f2_unpack(x01, x0, x1);
-                        p01 = f2_pack(ex2_approx(x0), ex2_approx(x1));
-                    }
+                    float x0, x1;
+                    f2_unpack(x01, x0, x1);
+                    const uint64_t p01 = f2_pack(ex2_approx(x0), ex2_approx(x1));
                     float p0, p1;
                     f2_unpack(p01, p0, p1);
                     pk[e] = pack_half2(p0, p1);
                     if (e & 1) l1 = f2_add(l1, p01);
                     else l0 = f2_add(l0, p01);
                 }
-                if (pingpong) mbar_arrive(&turn[1 - t]);
                 float l_lo, l_hi;
                 f2_unpack(f2_add(l0, l1), l_lo, l_hi);
                 A4_TRACE(5);

@@ -36,16 +36,6 @@ namespace star {
 
 STAR_DEVINL uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-STAR_DEVINL bool elect_one() {
-    uint32_t pred = 0;
-    asm volatile(
-        "{\n\t.reg .pred P;\n\t"
-        "elect.sync _|P, 0xffffffff;\n\t"
-        "selp.b32 %0, 1, 0, P;\n\t}\n"
-        : "=r"(pred));
-    return pred != 0;
-}
-
 // ---------------------------------------------------------------- mbarrier
 STAR_DEVINL void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
@@ -142,15 +132,6 @@ STAR_DEVINL void tmem_ld32(uint32_t taddr, uint32_t* r) {
           "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
           "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
           "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-}
-// 32 lanes x 16 columns
-STAR_DEVINL void tmem_ld16(uint32_t taddr, uint32_t* r) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
         : "r"(taddr));
 }
 STAR_DEVINL void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
@@ -258,14 +239,6 @@ STAR_DEVINL void tmem_st32(uint32_t taddr, const uint32_t* r) {
         "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
         : "memory");
 }
-STAR_DEVINL void tmem_st16(uint32_t taddr, const uint32_t* r) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-        : "memory");
-}
 STAR_DEVINL void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 STAR_DEVINL void unpack8h(const uint4& u, float* f) {
@@ -282,19 +255,6 @@ STAR_DEVINL float ex2_approx(float x) {
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
-}
-// 2^x on the FMA/ALU pipes (no MUFU): round-to-nearest split x = i + f, f in [-0.5, 0.5], degree-3 minimax
-// polynomial for 2^f (max rel. error 7.7e-5, below the fp16 rounding of the probabilities), exponent inserted
-// with one integer add.  Valid for x in [-126, 126].
-STAR_DEVINL float ex2_poly(float x) {
-    x = fmaxf(x, -126.0f);
-    const float magic = 12582912.0f;                 // 1.5 * 2^23
-    const float fr = __fadd_rn(x, magic);            // integer part lands in the low mantissa bits
-    const float f = __fsub_rn(x, __fsub_rn(fr, magic));
-    float p = fmaf(0.05508868396282196f, f, 0.24260404706001282f);
-    p = fmaf(p, f, 0.6932762265205383f);
-    p = fmaf(p, f, 0.9999289512634277f);
-    return __int_as_float(__float_as_int(p) + (__float_as_int(fr) << 23));
 }
 
 // ---- packed fp32x2 arithmetic (sm_100: FFMA2 / FADD2, one issue slot for two lanes' worth of work) ----
@@ -320,22 +280,5 @@ STAR_DEVINL uint64_t f2_add(uint64_t a, uint64_t b) {
     uint64_t r;
     asm("add.rn.ftz.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
     return r;
-}
-// ex2_poly on a packed pair
-STAR_DEVINL uint64_t ex2_poly2(uint64_t x) {
-    float x0, x1;
-    f2_unpack(x, x0, x1);
-    x = f2_pack(fmaxf(x0, -126.0f), fmaxf(x1, -126.0f));
-    const uint64_t fr = f2_add(x, f2_pack(12582912.0f, 12582912.0f));
-    const uint64_t t = f2_add(fr, f2_pack(-12582912.0f, -12582912.0f));
-    const uint64_t f = f2_fma(t, f2_pack(-1.0f, -1.0f), x);
-    uint64_t q = f2_fma(f2_pack(0.05508868396282196f, 0.05508868396282196f), f, f2_pack(0.24260404706001282f, 0.24260404706001282f));
-    q = f2_fma(q, f, f2_pack(0.6932762265205383f, 0.6932762265205383f));
-    q = f2_fma(q, f, f2_pack(0.9999289512634277f, 0.9999289512634277f));
-    float q0, q1, r0, r1;
-    f2_unpack(q, q0, q1);
-    f2_unpack(fr, r0, r1);
-    return f2_pack(__int_as_float(__float_as_int(q0) + (__float_as_int(r0) << 23)),
-                   __int_as_float(__float_as_int(q1) + (__float_as_int(r1) << 23)));
 }
 }  // namespace star

@@ -31,9 +31,8 @@ int g_sms[STAR_MAX_DEVICES] = {0};            // SM count per initialised device
 constexpr int kWideWastePct = 10;             // largest padding (percent of N) accepted for the 128x256 tiles ...
 constexpr int kWideWasteLongKPct = 25;        // ... and for reductions >= 1920 (N = 640 as 3 x 256: +16 % on the 640-channel convs)
 constexpr int kWideMinK = 256;                // smallest reduction length that takes the 128x256 tiles
-#ifndef STAR_GEMM_DBUF_MAXK
-#define STAR_GEMM_DBUF_MAXK 700               // 128x256-tile GEMMs with reductions up to this length use two output staging buffers
-#endif                                        // (A/B: profiles/r02_kbench_gemm_dbuf_ab.log -- qkv -5 %, 512->1536 -9 %, longer K / narrower tiles lose)
+constexpr int kDbufMaxK = 700;                // 128x256-tile GEMMs with reductions up to this length use two output staging buffers
+                                              // (A/B: profiles/r02_kbench_gemm_dbuf_ab.log -- qkv -5 %, 512->1536 -9 %, longer K / narrower tiles lose)
 std::atomic<long long> g_launches{0};
 
 // SM count of the CURRENT device (kernels are launched on the caller's current device / stream)
@@ -115,11 +114,13 @@ struct TapDesc {
     void* out;
 };
 
+// Shared by both tap-GEMM kernels: the kernel parameters, the number of M tiles, and the tensor maps of the input view (A)
+// and of the weights (W, BN rows per box; GEGLU: BN / 2 value rows and BN / 2 gate rows).  `name` prefixes the error message.
 template <int BN>
-int launch_tapgemm_bn(const TapDesc& d, cudaStream_t st) {
-    TapGemmParams p;
+int tapgemm_setup(const TapDesc& d, const char* name, TapGemmParams& p, long long& m_tiles, CUtensorMap& ta,
+                  CUtensorMap& tw) {
     memset(&p, 0, sizeof(p));
-    long long m_tiles = 1;
+    m_tiles = 1;
     int box_rows = 1;
     for (int i = 0; i < 4; ++i) {
         p.on[i] = d.on[i];
@@ -128,57 +129,7 @@ int launch_tapgemm_bn(const TapDesc& d, cudaStream_t st) {
         m_tiles *= p.tiles[i];
         box_rows *= d.box[i];
     }
-    if (box_rows > TG_BM) return fail("tapgemm: box has %d rows (> %d)", box_rows, TG_BM);
-    p.box_rows = box_rows;
-    p.ntaps = d.ntaps;
-    memcpy(p.tap, d.tap, sizeof(p.tap));
-    p.K = d.K;
-    p.k_chunks = (d.K + TG_BK - 1) / TG_BK;
-    p.N = d.N;
-    p.flags = d.flags;
-    p.bias = (const __half*)d.bias;
-    p.rowvec = (const __half*)d.rowvec;
-    p.rowvec_div = (int)std::max(1ll, d.rowvec_div);
-    p.rowvec_ld = d.ldrowvec > 0 ? d.ldrowvec : d.N;
-    p.residual = (const __half*)d.residual;
-    p.res_ld = d.ldres;
-    p.out = (__half*)d.out;
-    p.out_ld = d.ldo;
-    const bool geglu = d.flags & TG_GEGLU;
-    if (geglu && BN != 128) return fail("tapgemm: GEGLU requires BN=128");
-    if (geglu && (d.N % 64)) return fail("tapgemm: GEGLU requires N %% 64 == 0 (N=%d)", d.N);
-    if (m_tiles > 65535) return fail("tapgemm: %lld M tiles exceed grid.y", m_tiles);
-
-    CUtensorMap ta, tw;
-    unsigned abox[5] = {TG_BK, (unsigned)d.box[0], (unsigned)d.box[1], (unsigned)d.box[2], (unsigned)d.box[3]};
-    if (make_tmap(&ta, d.A, 5, d.adim, d.astr, abox)) return 1;
-    const unsigned long long wrows = geglu ? 2ull * d.N : (unsigned long long)d.N;
-    unsigned long long wdim[2] = {(unsigned long long)d.ntaps * d.K, wrows};
-    unsigned long long wstr[2] = {1, (unsigned long long)d.ntaps * d.K};
-    unsigned wbox[2] = {TG_BK, (unsigned)(geglu ? BN / 2 : BN)};
-    if (make_tmap(&tw, d.W, 2, wdim, wstr, wbox)) return 1;
-
-    const int n_per_tile = geglu ? BN / 2 : BN;
-    dim3 grid((d.N + n_per_tile - 1) / n_per_tile, (unsigned)m_tiles, 1);
-    tapgemm_kernel<BN><<<grid, TG_THREADS, TapGemmSmem<BN>::TOTAL, st>>>(ta, tw, p);
-    STAR_LAUNCH_CHECK("tapgemm");
-    return 0;
-}
-
-template <int BN>
-int launch_tapgemm2_bn(const TapDesc& d, cudaStream_t st) {
-    TapGemmParams p;
-    memset(&p, 0, sizeof(p));
-    long long m_tiles = 1;
-    int box_rows = 1;
-    for (int i = 0; i < 4; ++i) {
-        p.on[i] = d.on[i];
-        p.box[i] = d.box[i];
-        p.tiles[i] = (d.on[i] + d.box[i] - 1) / d.box[i];
-        m_tiles *= p.tiles[i];
-        box_rows *= d.box[i];
-    }
-    if (box_rows > TG_BM) return fail("tapgemm2: box has %d rows (> %d)", box_rows, TG_BM);
+    if (box_rows > TG_BM) return fail("%s: box has %d rows (> %d)", name, box_rows, TG_BM);
     p.box_rows = box_rows;
     p.ntaps = d.ntaps;
     memcpy(p.tap, d.tap, sizeof(p.tap));
@@ -195,6 +146,41 @@ int launch_tapgemm2_bn(const TapDesc& d, cudaStream_t st) {
     p.res_ld = d.ldres;
     p.out = (__half*)d.out;
     p.out_ld = d.ldo;
+
+    const bool geglu = d.flags & TG_GEGLU;
+    unsigned abox[5] = {TG_BK, (unsigned)d.box[0], (unsigned)d.box[1], (unsigned)d.box[2], (unsigned)d.box[3]};
+    if (make_tmap(&ta, d.A, 5, d.adim, d.astr, abox)) return 1;
+    const unsigned long long wrows = geglu ? 2ull * d.N : (unsigned long long)d.N;
+    unsigned long long wdim[2] = {(unsigned long long)d.ntaps * d.K, wrows};
+    unsigned long long wstr[2] = {1, (unsigned long long)d.ntaps * d.K};
+    unsigned wbox[2] = {TG_BK, (unsigned)(geglu ? BN / 2 : BN)};
+    return make_tmap(&tw, d.W, 2, wdim, wstr, wbox);
+}
+
+template <int BN>
+int launch_tapgemm_bn(const TapDesc& d, cudaStream_t st) {
+    TapGemmParams p;
+    long long m_tiles;
+    CUtensorMap ta, tw;
+    if (tapgemm_setup<BN>(d, "tapgemm", p, m_tiles, ta, tw)) return 1;
+    const bool geglu = d.flags & TG_GEGLU;
+    if (geglu && BN != 128) return fail("tapgemm: GEGLU requires BN=128");
+    if (geglu && (d.N % 64)) return fail("tapgemm: GEGLU requires N %% 64 == 0 (N=%d)", d.N);
+    if (m_tiles > 65535) return fail("tapgemm: %lld M tiles exceed grid.y", m_tiles);
+
+    const int n_per_tile = geglu ? BN / 2 : BN;
+    dim3 grid((d.N + n_per_tile - 1) / n_per_tile, (unsigned)m_tiles, 1);
+    tapgemm_kernel<BN><<<grid, TG_THREADS, TapGemmSmem<BN>::TOTAL, st>>>(ta, tw, p);
+    STAR_LAUNCH_CHECK("tapgemm");
+    return 0;
+}
+
+template <int BN>
+int launch_tapgemm2_bn(const TapDesc& d, cudaStream_t st) {
+    TapGemmParams p;
+    long long m_tiles;
+    CUtensorMap ta, tw, to, tr;
+    if (tapgemm_setup<BN>(d, "tapgemm2", p, m_tiles, ta, tw)) return 1;
     const bool geglu = d.flags & TG_GEGLU;
     const int n_per_tile = geglu ? BN / 2 : BN;
     TapGemm2Extra ex;
@@ -203,14 +189,6 @@ int launch_tapgemm2_bn(const TapDesc& d, cudaStream_t st) {
     if (total > 0x7fffffffll) return fail("tapgemm2: too many tiles");
     ex.num_tiles = (int)total;
 
-    CUtensorMap ta, tw, to, tr;
-    unsigned abox[5] = {TG_BK, (unsigned)d.box[0], (unsigned)d.box[1], (unsigned)d.box[2], (unsigned)d.box[3]};
-    if (make_tmap(&ta, d.A, 5, d.adim, d.astr, abox)) return 1;
-    const unsigned long long wrows = geglu ? 2ull * d.N : (unsigned long long)d.N;
-    unsigned long long wdim[2] = {(unsigned long long)d.ntaps * d.K, wrows};
-    unsigned long long wstr[2] = {1, (unsigned long long)d.ntaps * d.K};
-    unsigned wbox[2] = {TG_BK, (unsigned)(geglu ? BN / 2 : BN)};
-    if (make_tmap(&tw, d.W, 2, wdim, wstr, wbox)) return 1;
     // output / residual: (N, n1..n4) with row pitch ld; 32-column boxes, SWIZZLE_64B staging tiles
     unsigned obox[5] = {32, (unsigned)d.box[0], (unsigned)d.box[1], (unsigned)d.box[2], (unsigned)d.box[3]};
     unsigned long long odim[5] = {(unsigned long long)d.N, (unsigned long long)d.on[0], (unsigned long long)d.on[1],
@@ -227,8 +205,7 @@ int launch_tapgemm2_bn(const TapDesc& d, cudaStream_t st) {
     if (make_tmap(&to, d.out, 5, odim, ostr, obox, CU_TENSOR_MAP_SWIZZLE_64B)) return 1;
     // Output staging depth.  Short reductions are epilogue-bound (the main loop alone runs at 75-82 % of peak, the serialised
     // store drain costs 25-30 %: profiles/r02_kbench_gemm_attribution.log) -> two staging buffers, one operand stage fewer.
-    ex.dbuf = ((long long)d.ntaps * d.K <= STAR_GEMM_DBUF_MAXK) ? 1 : 0;
-    ex.res_direct = 0;
+    ex.dbuf = ((long long)d.ntaps * d.K <= kDbufMaxK) ? 1 : 0;
     const bool res_tma = d.residual && TapGemm2Smem<BN>::RES_TMA;
     if (ex.dbuf && TapGemm2Smem<BN>::stages(res_tma, true) < 3) ex.dbuf = 0;       // BN = 160 + residual: no room for a second buffer
     if (res_tma) {

@@ -17,13 +17,7 @@
 #include "common.cuh"
 #include "tapgemm.cuh"
 
-// Attribution experiments (tools/build_variant.py -DSTAR_GEMM_EXP=n; the shipped library is n = 0):
-//   1: the epilogue computes and stages but never issues its TMA stores      -> time without the store path
-//   2: the epilogue only drains TMEM (no bias / activation math, no staging)  -> time of loads + MMA alone
-#ifndef STAR_GEMM_EXP
-#define STAR_GEMM_EXP 0
-#endif
-
+// Instrumented build (tools/build_variant.py -DSTAR_GEMM_TRACE=1):
 //   STAR_GEMM_TRACE 1: CTA 0 records clock64() timestamps of its producer / MMA / epilogue roles per tile into g_tg2_trace
 //                     (tools/gemm_trace.py reads it back through star_debug_read_trace); never set in the shipped library.
 #ifndef STAR_GEMM_TRACE
@@ -91,7 +85,6 @@ struct TapGemm2Extra {
     int dbuf;             // 1: two output staging buffers -- the TMA-store drain of pass i overlaps the arithmetic of pass i+1
                           //    (attribution, profiles/r02_kbench_gemm_attribution.log: with one buffer the short-K GEMMs lose
                           //    25-30 % to the serialised drain)
-    int res_direct;       // 1: read the residual with direct 16-byte loads even where this BN would prefetch it by TMA
 };
 
 // EPI selects a compile-time specialisation of the epilogue (the role timeline showed the generic epilogue -- ~1 500 SASS
@@ -115,7 +108,7 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
     const int OFF_RES = OFF_OUT + SM::OUT_BYTES * (ex.dbuf ? 2 : 1);
     constexpr bool GEN = EPI == TG2_EPI_GENERIC;
     // residual tile prefetched by TMA (else: direct loads)
-    const bool res_tma = EPI == TG2_EPI_RES ? true : (GEN && SM::RES_TMA && p.residual != nullptr && !ex.res_direct);
+    const bool res_tma = EPI == TG2_EPI_RES ? true : (GEN && SM::RES_TMA && p.residual != nullptr);
     const int OFF_BAR = OFF_RES + (res_tma ? SM::OUT_BYTES : 0);
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + OFF_BAR);
     uint64_t* empty_bar = full_bar + TG2_MAX_STAGES;
@@ -276,7 +269,7 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                     mbar_wait(&stage_full[ob], use & 1);
 #pragma unroll 1
                     for (int sb = 0; sb < (pass_end - pass0) / 32; ++sb) {
-                        if (STAR_GEMM_EXP == 0 && n_base + pass0 + sb * 32 < p.N)
+                        if (n_base + pass0 + sb * 32 < p.N)
                             tma_store_5d(&tmap_out, smem + OFF_OUT + ob * SM::OUT_BYTES + sb * 8192, n_base + pass0 + sb * 32,
                                          org[0], org[1], org[2], org[3]);
                     }
@@ -348,15 +341,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                 float f[32];
                 tmem_ld32(t_row + c0, v);
                 const int n0 = n_base + c0;
-#if STAR_GEMM_EXP == 2
-                tmem_ld_wait();
-                if (c0 == last_c0) {
-                    tc_fence_before();
-                    mbar_arrive(&acc_empty[buf]);
-                }
-                if (v[0] == 0x12345678u) out_row[0] = 1;          // keep the load alive
-                continue;
-#endif
                 if (geglu) {
                     uint32_t g[32];
                     tmem_ld32(t_row + (BN / 2) + c0, g);

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Build an A/B variant of libstar_sm100.so with extra -D macros (compile-time experiment knobs documented in the kernels'
-headers), e.g.   python tools/build_variant.py pp1 -DSTAR_ATTN_PINGPONG=1
+"""Build a variant of libstar_sm100.so with extra -D macros (the instrumented trace builds documented in the kernels'
+headers), e.g.   python tools/build_variant.py gtrace -DSTAR_GEMM_TRACE=1
 The variant lands in tools/variants/libstar_<tag>.so (git-ignored, travels to the GPU box); tools/kbench.py --lib <path>
 and bench.py --lib <path> load it instead of the shipped library.  The product has no run-time kernel dispatch."""
 import os
